@@ -16,7 +16,11 @@ cache.  tokens = sessions * (seq + decode).
                  oracle port on all host threads (pinned with threadpoolctl), bounded sample; --cpu-impl hf switches to
                  HF transformers on torch CPU, which measured 30x slower on the GPU box (profiles/r02c_reference_hf.json)
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload llama8b|bge|pack]
+  --dump-outputs DIR : after the timed steps, what the last one returned to the caller as DIR/<name>.npy (float32 /
+                 float64, 64 MB in all, a seeded row sample beyond that); inputs are seeded, so two builds compare output
+                 for output
+
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload llama8b|bge|pack] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -110,18 +114,37 @@ def session_prompt(global_index, seq, vocab):
 
 
 def serve_once(e, hb, prompts, decode):
-    """All sessions through the public C-ABI path; returns generated token count."""
+    """All sessions through the public C-ABI path; returns each session's generated token ids."""
     sp = hb.Sampling(max_tokens=decode, temperature=0.0)
     rids = [e.submit(p, sp) for p in prompts]
-    got = 0
+    outs = []
     for r in rids:
-        fin = 0
+        got, fin = [], 0
         while not fin:
             e.wait(r, 60000)
             toks, fin = e.poll(r)
-            got += len(toks)
+            got += toks
         e.release(r)
-    return got
+        outs.append(got)
+    return outs
+
+
+DUMP_BYTES = 64 * 10 ** 6   # everything one --dump-outputs writes, .npy headers included
+
+
+def dump_outputs(path, outputs, budget=DUMP_BYTES):
+    """--dump-outputs: each array of `outputs` as path/<name>.npy.  An array over its share of `budget` is cut to a fixed,
+    seeded sample of its rows (same rows on every run of the same arguments), whose indices go to path/<name>_rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    share = budget // len(outputs) - 2 * 128   # room for the array and its row indices, less two .npy headers
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if a.nbytes > share:
+            keep = share // (a[0].nbytes + 8)
+            rows = np.sort(np.random.default_rng(0).choice(len(a), size=keep, replace=False)).astype(np.float64)
+            np.save(os.path.join(path, name + "_rows.npy"), rows)
+            a = a[rows.astype(np.int64)]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def serve_latency(e, hb, prompts, decode, spread_s=0.0):
@@ -349,6 +372,8 @@ def bench_bge(args):
     wall = (time.perf_counter() - t0) / args.steps
     s1 = e.stats()
     clocks = sampler.stop()
+    if args.dump_outputs:   # before the profiled pass below reuses `out`
+        dump_outputs(args.dump_outputs, {"embeddings": out})   # the last timed step's fp32 vectors [chunk, hidden]
     dev = (s1["gpu_ms_prefill"] - s0["gpu_ms_prefill"]) / args.steps / 1e3
     e.set_profile(True)
     p0 = e.stats()
@@ -434,7 +459,7 @@ def bench_pack(args):
         prompts = [rng.integers(0, desc.vocab, size=prompt).astype(np.int32) for _ in range(sessions)]
         toks, t0 = 0, time.perf_counter()
         while time.perf_counter() - t0 < seconds:
-            toks += serve_once(e, hb, prompts, decode) + sessions * prompt
+            toks += sum(map(len, serve_once(e, hb, prompts, decode))) + sessions * prompt
         out[key] = toks / (time.perf_counter() - t0)
 
     def embed_load(e, desc, chunks, out, key):
@@ -521,7 +546,13 @@ def main():
     ap.add_argument("--pack-seconds", type=float, default=8.0)
     ap.add_argument("--pack-sms", type=int, nargs=3, default=[96, 24, 24], help="SM shares of 8B / 1B / bge")
     ap.add_argument("--pack-modes", nargs="+", default=["none", "budget", "partition"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (llama8b: tokens, bge: embeddings)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.workload == "pack"):
+        ap.error("--dump-outputs: native llama8b and bge workloads only")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -587,7 +618,7 @@ def main():
     e.start()
     for _ in range(args.warmup):
         got = serve_once(e, hb, prompts, args.decode)
-        assert got == args.sessions * args.decode
+        assert sum(map(len, got)) == args.sessions * args.decode
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
     barrier()
@@ -596,7 +627,7 @@ def main():
     s0 = e.stats()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        serve_once(e, hb, prompts, args.decode)
+        outs = serve_once(e, hb, prompts, args.decode)
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
     s1 = e.stats()
@@ -735,6 +766,10 @@ def main():
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_field(args.cpu_impl)
         print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        # what a client of hb_submit / hb_poll received in the last timed step: greedy token ids [session, decode step]
+        dump_outputs(args.dump_outputs, {"tokens" + (f"_rank{rank}" if world > 1 else ""): np.array(outs, np.float64)},
+                     DUMP_BYTES // world)
     e.close()
     if world > 1:
         dist.destroy_process_group()
